@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this framework (one process per GPU; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm's CPU path (oracle port) on host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    # + what the last timed step computed, as DIR/*.npy
 
 One "step" = hint-encoder fwd + SD-1.5 UNet fwd + MSE + backward (dX, LoRA dA/dB, hint-encoder dW) + gradient
 all-reduce (N > 1) + clip_grad_norm + AdamW, on synthetic 512x512 inputs (64x64 latents, 77x768 text states), batch 8
@@ -23,6 +24,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 METRIC = "train_images_per_sec_512px_bs8_per_gpu"
 UNIT = "images/s"
@@ -56,6 +58,10 @@ def parse():
     ap.add_argument("--no-aux", action="store_true", help="skip the auxiliary numbers (denoise C3/C5, drop-in path, per-shape GEMM table)")
     ap.add_argument("--aux-only", default=None, choices=["train_from_pixels"],
                     help="run ONE auxiliary measurement in this process and print its JSON (bench.py runs it as an isolated child process)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, gradient norm, parameters and AdamW moments "
+                         "after the update) as float32 DIR/<name>.npy; the inputs and initial weights are seeded, so two builds can be "
+                         "compared output for output")
     return ap.parse_args()
 
 
@@ -459,6 +465,28 @@ def aux_gemm_table(torch, ops):
 
 
 # ------------------------------------------------------------------------------------------------------ GPU arm
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, tr, loss):
+    """What one Trainer.step leaves its caller: the loss, the global gradient norm before clipping, and the trainable parameters
+    and AdamW moments after the update, as float32 .npy files under out_dir.  A parameter arena whose three arrays would exceed
+    DUMP_BUDGET_BYTES is written as one fixed, seeded sample of its elements: the sorted first k of
+    torch.randperm(numel, generator=torch.Generator().manual_seed(0)), the same elements in all three files."""
+    import numpy as np
+    import torch
+
+    n = tr.numel
+    k = min(n, (DUMP_BUDGET_BYTES - 1024) // (3 * 4))        # three float32 arrays; 1 KiB for the two scalars and the .npy headers
+    idx = None if k == n else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values.to(tr.flat_p.device)
+    arrays = {"loss": loss.reshape(-1), "grad_norm": tr.gnorm_sq.sqrt().reshape(-1) * tr.arena.grad_scale}
+    for name, t in (("params", tr.flat_p), ("exp_avg", tr.flat_m), ("exp_avg_sq", tr.flat_v)):
+        arrays[name] = t[:n] if idx is None else t[:n][idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -477,6 +505,7 @@ def run_ours(a):
     dev = torch.device("cuda", local)
     B = a.batch
     unet = cb.UNet2DConditionModel.synthetic(dev, seed=0)
+    torch.manual_seed(0)        # the ControlLoRA's default initialisation: the same weights on every run
     cl = cb.ControlLoRA.from_config(NAMED[a.config]).to(dev)
     g = torch.Generator().manual_seed(3)
     with torch.no_grad():       # LoRA `up` weights are zero-initialised: give them values so no path is trivially dead
@@ -516,6 +545,8 @@ def run_ours(a):
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, tr, loss)      # before the end-to-end and roofline passes below train further
     launches = (_lib.launch_count() - n0) // max(a.steps, 1)
     if tr.cuda_graph and tr.launches_per_step:
         launches = tr.launches_per_step      # kernels inside the replayed graph (counted at capture) + optimizer launches

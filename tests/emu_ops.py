@@ -672,6 +672,12 @@ def install() -> None:
         return
     import os
 
+    # The real wrappers run on CPU tensors and count on the launcher failing at its first CUDA call.  On a machine with a GPU that
+    # call would succeed and launch kernels on host pointers, so host-logic mode hides every device from the process; it has to be
+    # installed before anything in the process has initialised CUDA.
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
+    if torch.cuda.device_count() != 0:
+        raise RuntimeError("host-logic mode (CLB_EMU=1) must be installed before the process initialises CUDA")
     _INSTALLED["env"] = os.environ.get("CLB_DRYRUN")
     os.environ["CLB_DRYRUN"] = "1"          # the package's require_cuda() guards accept CPU tensors in host-logic mode only
     g = globals()

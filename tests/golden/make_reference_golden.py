@@ -32,6 +32,12 @@ CASES = {
     "concat": (dict(lora_concat_hidden=True, lora_control_rank=32, lora_pre_conv_skipped=True, lora_control_self_add=False), False, 1.0),
 }
 OUT = Path(__file__).resolve().parent / "reference_models.pt"
+GRAD_STRIDE = 3          # every third element of each kept gradient is stored: keeps the file under 1 MB
+
+
+def grad_sample(g: torch.Tensor) -> torch.Tensor:
+    """The stored elements of a gradient tensor (flattened, at GRAD_STRIDE)."""
+    return g.detach().float().cpu().reshape(-1)[::GRAD_STRIDE]
 
 
 def seeded_state(case):
@@ -98,7 +104,7 @@ def run_front_half(M, case):
         if p.grad is None:
             continue
         norms[n] = p.grad.double().norm().float()
-        if p.numel() <= 1024 and (n.startswith("lora_layers.") or p.dim() <= 1):     # adapter / control matrices, biases, norm parameters: in full
+        if p.numel() <= 1024 and (n.startswith("lora_layers.") or p.dim() <= 1):     # adapter / control matrices, biases, norm parameters
             small[n] = p.grad.detach().clone()
     for name, op in stacked.items():
         for n, p in op.named_parameters():
@@ -106,18 +112,20 @@ def run_front_half(M, case):
                 small[f"pre_lora::{name}::{n}"] = p.grad.detach().clone()
     # one flat tensor + an index per dictionary (a pickle of ~1000 tiny tensors is mostly per-tensor overhead)
     out["grads"] = {"names": list(small), "shapes": [tuple(v.shape) for v in small.values()],
-                    "flat": torch.cat([v.reshape(-1) for v in small.values()])}
+                    "flat": torch.cat([grad_sample(v) for v in small.values()])}
     out["grad_norms"] = {"names": list(norms), "values": torch.stack(list(norms.values()))}
     return out
 
 
 def unpack_grads(packed) -> dict:
+    """name -> the stored sample (grad_sample) of that gradient; "shapes" are the shapes of the whole tensors."""
     out, off = {}, 0
     for n, shp in zip(packed["names"], packed["shapes"]):
         k = 1
         for d in shp:
             k *= d
-        out[n] = packed["flat"][off:off + k].view(shp)
+        k = -(-k // GRAD_STRIDE)
+        out[n] = packed["flat"][off:off + k]
         off += k
     return out
 

@@ -1,10 +1,10 @@
-"""Pins the oracle restatement of the reference's own code (oracle/models_ref.py <- /root/reference/models.py) to the REAL file:
-models.py is imported unmodified (tests/golden/reference_import.py stands in for the ten `diffusers` names it imports) and run next
-to the restatement on the same weights and inputs - every shipped config's hint encoder, every processor class (plain / v1 / V2 /
-post_add / concat_hidden / stacked chains / scale != 1), and a whole tiny UNet with the reference's processors installed.
-Runs where /root/reference exists (this container); on the GPU box the committed golden vectors generated from the same import
-(tests/golden/reference_models.pt, tests/golden/make_reference_golden.py) take over: the oracle against them on the CPU, the CUDA
-path against them under `-m gpu`."""
+"""Pins the oracle restatement of the reference's own code (oracle/models_ref.py <- the reference's models.py) to what that code
+computes: every shipped config's hint encoder, every processor class (plain / v1 / V2 / post_add / concat_hidden / stacked chains /
+scale != 1), and a whole tiny UNet with the reference's processors installed.  The reference's outputs were computed by its
+models.py, imported unmodified (tests/golden/reference_import.py stands in for the ten `diffusers` names it imports), on weights
+seeded through the oracle classes, and are stored in tests/golden/reference_pin.pt (tests/golden/make_reference_pin.py); the
+tests rebuild the same weights and inputs and run the restatement on them.  The golden vectors of the training-step front half
+(tests/golden/reference_models.pt, tests/golden/make_reference_golden.py) pin the oracle here and the CUDA path under `-m gpu`."""
 import sys
 from pathlib import Path
 
@@ -14,8 +14,7 @@ import torch
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 from oracle import models_ref as MR  # noqa: E402
-from oracle import unet_ref as UR  # noqa: E402
-from tests.golden import reference_import as RI  # noqa: E402
+from tests.golden import make_reference_pin as P  # noqa: E402
 
 @pytest.fixture(autouse=True)
 def _single_thread():
@@ -27,182 +26,67 @@ def _single_thread():
     torch.set_num_threads(n)
 
 
-needs_reference = pytest.mark.skipif(not RI.available(), reason="/root/reference is not present on this machine")
-CONFIGS = ["base", "fill50k", "diffusiondb-canny", "mpii-pose", "diffusiondb-canny-v2", "mpii-pose-v2", "post-add", "danbooru-sketch"]
+GOLD = P.load()
 
 
-def _randomize_(m, seed):
-    g = torch.Generator().manual_seed(seed)
-    with torch.no_grad():
-        for n, p in m.named_parameters():
-            if n.endswith("up.weight"):
-                p.copy_(0.05 * torch.randn(p.shape, generator=g))
-            elif "norm" in n:
-                p.add_(0.1 * torch.randn(p.shape, generator=g))
+def _close(have, want, tol, floor=0.0):
+    """Two digests of the same tensor (shape, strided sample, fp64 norm; tests/golden/make_reference_pin.py): the sampled
+    elements within tol x the largest sampled magnitude (+ floor), and the norm of the whole tensor within tol (+ floor)."""
+    return (have["shape"] == want["shape"] and have["sample"].shape == want["sample"].shape
+            and float((have["sample"] - want["sample"]).abs().max()) <= tol * float(want["sample"].abs().max()) + floor
+            and abs(have["norm"] - want["norm"]) <= tol * want["norm"] + floor)
 
 
-@needs_reference
-@pytest.mark.parametrize("name", CONFIGS)
+@pytest.mark.parametrize("name", P.CONFIGS)
 def test_hint_encoder_restatement_equals_the_reference(name):
     """ControlLoRA.__init__ wiring + forward (models.py:618-835) for every shipped configs/*.json: same state-dict keys / shapes,
-    and - on the reference's weights - bit-comparable control states and parameter gradients."""
-    R = RI.reference_models()
-    cfg = RI.reference_config(name)
-    torch.manual_seed(0)
-    ref = R.ControlLoRA(**cfg)
-    _randomize_(ref, 1)
-    ora = MR.ControlLoRA.from_config(cfg)
-    assert list(ora.state_dict().keys()) == list(ref.state_dict().keys())
-    ora.load_state_dict(ref.state_dict())
-    assert [[type(p).__name__ for p in lvl] for lvl in ora.lora_layers] == [[type(p).__name__ for p in lvl] for lvl in ref.lora_layers]
-    for po, pr in zip([p for lvl in ora.lora_layers for p in lvl], [p for lvl in ref.lora_layers for p in lvl]):
-        for attr in ("hidden_size", "cross_attention_dim", "rank", "post_add", "concat_hidden", "control_self_add",
-                     "key_states_skipped", "value_states_skipped", "output_states_skipped"):
-            assert getattr(po, attr) == getattr(pr, attr), attr
-    g = torch.Generator().manual_seed(2)
-    guide = torch.rand(1, 3, 64, 64, generator=g) * 2 - 1
-    so, sr = ora(guide).control_states, ref(guide).control_states
-    ws = [torch.randn(s.shape, generator=g) for s in sr]
-    sum((s * w).sum() for s, w in zip(so, ws)).backward()
-    sum((s * w).sum() for s, w in zip(sr, ws)).backward()
-    for a, b in zip(so, sr):
-        assert a.shape == b.shape and float((a - b).abs().max()) <= 1e-4 * float(b.abs().max())
-    for (n, a), (_, b) in zip(ora.named_parameters(), ref.named_parameters()):
-        if b.grad is None:
-            assert a.grad is None, n
+    same processor classes and flags, and - on the same seeded weights - the control states and parameter gradients the
+    reference computed."""
+    gold = GOLD["hint_encoder_outputs"][GOLD["hint_encoder"][name]]
+    got = P.hint_encoder_case(MR, GOLD["configs"][name])
+    assert got["keys"] == gold["keys"]
+    assert got["proc_types"] == gold["proc_types"]
+    assert got["proc_attrs"] == gold["proc_attrs"]
+    assert got["injected"]
+    assert len(got["states"]) == len(gold["states"])
+    for i, (a, b) in enumerate(zip(got["states"], gold["states"])):
+        assert _close(a, b, 1e-4), f"control state {i}"
+    assert list(got["grads"]) == list(gold["grads"])
+    for n, b in gold["grads"].items():
+        a = got["grads"][n]
+        if b is None:
+            assert a is None, n
         else:
-            assert float((a.grad - b.grad).abs().max()) <= 1e-3 * float(b.grad.abs().max()) + 1e-9, n
-    # the processors received the same injected tensors (models.py:826-829)
-    for lo, lr, s in zip(ora.lora_layers, ref.lora_layers, sr):
-        for po, pr in zip(lo, lr):
-            assert torch.equal(pr.control_states, s) and po.control_states.shape == s.shape
+            assert a is not None and _close(a, b, 1e-3, 1e-9), n
 
 
-def _proc_pair(R, cls, C, xd, seed, **kw):
-    ref = getattr(R, cls)(C, xd, **kw)
-    _randomize_(ref, seed)
-    ora = getattr(MR, cls)(C, xd, **kw)
-    ora.load_state_dict(ref.state_dict())
-    return ref, ora
-
-
-PROC_CASES = {
-    "plain_self": ("LoRACrossAttnProcessor", False, {}, None, 1.0),
-    "plain_cross_post_add": ("LoRACrossAttnProcessor", True, dict(post_add=True), None, 0.7),
-    "plain_skips": ("LoRACrossAttnProcessor", True, dict(key_states_skipped=True, output_states_skipped=True), None, 1.0),
-    "v1_self": ("ControlLoRACrossAttnProcessor", False, {}, None, 1.0),
-    "v1_cross_scale": ("ControlLoRACrossAttnProcessor", True, dict(control_rank=8), None, 0.5),
-    "v1_post_add": ("ControlLoRACrossAttnProcessor", False, dict(post_add=True), None, 1.0),
-    "v1_concat": ("ControlLoRACrossAttnProcessor", True, dict(concat_hidden=True, control_rank=16, control_channels=96), None, 1.0),
-    "v1_stacked_pre_post": ("ControlLoRACrossAttnProcessor", True, {}, "plain", 0.5),
-    "v1_stacked_control": ("ControlLoRACrossAttnProcessor", False, {}, "control", 0.8),
-    "v2_self": ("ControlLoRACrossAttnProcessorV2", False, dict(control_channels=96), None, 1.0),
-    "v2_cross_scale": ("ControlLoRACrossAttnProcessorV2", True, dict(control_channels=96, control_rank=8), None, 0.6),
-    "v2_stacked": ("ControlLoRACrossAttnProcessorV2", False, dict(control_channels=96), "plain", 1.0),
-    "v2_stacked_control": ("ControlLoRACrossAttnProcessorV2", True, dict(control_channels=96), "control", 0.9),
-}
-
-
-@needs_reference
-@pytest.mark.parametrize("case", list(PROC_CASES))
+@pytest.mark.parametrize("case", list(P.PROC_CASES))
 def test_processor_restatement_equals_the_reference(case):
     """One processor call (models.py:118-152 / 222-287 / 357-431) on the same attention module, hidden states, text states and
-    control states: output, d hidden, every parameter gradient, d control - reference code vs restatement."""
-    R = RI.reference_models()
-    cls, cross, kw, stack, scale = PROC_CASES[case]
-    C, XD, H = 64, 48, 4
-    xd = XD if cross else None
-    torch.manual_seed(3)
-    attn = UR.CrossAttention(C, xd, H, C // H)
-    ref, ora = _proc_pair(R, cls, C, xd, 5, **kw)
-    extra = []
-    if stack == "plain":
-        a = _proc_pair(R, "LoRACrossAttnProcessor", C, xd, 7, rank=2, post_add=True)
-        b = _proc_pair(R, "LoRACrossAttnProcessor", C, xd, 8, rank=3)
-        ref.inject_pre_lora(a[0]); ora.inject_pre_lora(a[1])
-        ref.inject_post_lora(b[0]); ora.inject_post_lora(b[1])
-        extra = [a, b]
-    elif stack == "control":
-        a = _proc_pair(R, cls, C, xd, 9, **kw)
-        ref.inject_pre_lora(a[0]); ora.inject_pre_lora(a[1])
-        extra = [a]
-    g = torch.Generator().manual_seed(11)
-    hs = torch.randn(2, 36, C, generator=g)
-    ehs = torch.randn(2, 9, XD, generator=g) if cross else None
-    w = torch.randn(2, 36, C, generator=g)
-    outs = []
-    for side, (proc, stacked) in enumerate(((ref, [e[0] for e in extra]), (ora, [e[1] for e in extra]))):
-        h = hs.clone().requires_grad_(True)
-        ctrls = []
-        for p in [proc] + ([s for s in stacked if hasattr(s, "inject_control_states")] if stack == "control" else []):
-            if hasattr(p, "inject_control_states"):
-                cc = p.to_control.down.weight.shape[1] - (C if getattr(p, "concat_hidden", False) else 0)
-                c = torch.randn(2, cc, 6, 6, generator=torch.Generator().manual_seed(13 + len(ctrls))).requires_grad_(True)
-                p.inject_control_states(c)
-                ctrls.append(c)
-        y = proc(attn, h, ehs, None, scale)
-        (y * w).sum().backward()
-        grads = {n: p.grad.clone() for n, p in proc.named_parameters() if p.grad is not None}
-        for i, s in enumerate(stacked):
-            grads.update({f"stack{i}.{n}": p.grad.clone() for n, p in s.named_parameters() if p.grad is not None})
-        outs.append((y.detach(), h.grad.clone(), grads, [c.grad.clone() for c in ctrls]))
-        attn.zero_grad()
-    (yr, dhr, gr, dcr), (yo, dho, go, dco) = outs
-
-    def close(a, b, what):
-        assert a.shape == b.shape and float((a - b).abs().max()) <= 2e-5 * float(b.abs().max()) + 1e-8, what
-
-    close(yo, yr, "output")
-    close(dho, dhr, "d hidden")
-    assert set(go) == set(gr)
-    for n in gr:
-        close(go[n], gr[n], n)
-    assert len(dco) == len(dcr) and (len(dcr) > 0) == hasattr(ref, "inject_control_states")
-    for a, b in zip(dco, dcr):
-        close(a, b, "d control")
+    control states: output, d hidden, every parameter gradient, d control - restatement vs what the reference code computed."""
+    gold = GOLD["processor"][case]
+    got = P.processor_case(MR, case)
+    close = lambda a, b: _close(a, b, 2e-5, 1e-8)
+    assert close(got["out"], gold["out"]), "output"
+    assert close(got["d_hidden"], gold["d_hidden"]), "d hidden"
+    assert set(got["grads"]) == set(gold["grads"])
+    for n, b in gold["grads"].items():
+        assert close(got["grads"][n], b), n
+    assert len(got["d_control"]) == len(gold["d_control"]) and (len(gold["d_control"]) > 0) == gold["has_control"] == got["has_control"]
+    for a, b in zip(got["d_control"], gold["d_control"]):
+        assert close(a, b), "d control"
 
 
-@needs_reference
-@pytest.mark.parametrize("variant", ["v1", "v2", "post_add", "concat"])
+@pytest.mark.parametrize("variant", list(P.UNET_VARIANTS))
 def test_unet_with_reference_processors_equals_unet_with_restated_processors(variant):
     """The whole training-step front half on a tiny SD-style UNet (the UNet restatement is the same on both sides): the reference's
     ControlLoRA + processors + the wiring of train_text_to_image_control_lora.py:469-487 against oracle/models_ref.py."""
-    from tests.check_unet import TINY, TINY_LORA
-
-    R = RI.reference_models()
-    kw = dict(TINY_LORA)
-    kw.update({"v1": {}, "v2": dict(lora_control_version=2, lora_pre_conv_skipped=True), "post_add": dict(lora_post_add=True),
-               "concat": dict(lora_concat_hidden=True, lora_control_rank=32, lora_pre_conv_skipped=True, lora_control_self_add=False)}[variant])
-    torch.manual_seed(0)
-    ref = R.ControlLoRA(**kw)
-    _randomize_(ref, 1)
-    ora = MR.ControlLoRA(**kw)
-    ora.load_state_dict(ref.state_dict())
-    unets = []
-    for cl in (ref, ora):
-        u = UR.UNet2DConditionModel(**TINY)
-        UR.init_synthetic_(u, seed=1)
-        u.requires_grad_(False)
-        MR.wire_processors(u, cl)
-        unets.append(u)
-    g = torch.Generator().manual_seed(4)
-    guide = torch.rand(2, 3, 128, 128, generator=g) * 2 - 1
-    x = torch.randn(2, 4, 16, 16, generator=g)
-    ehs = torch.randn(2, 77, TINY["cross_attention_dim"], generator=g)
-    tgt = torch.randn(2, 4, 16, 16, generator=g)
-    t = torch.tensor([10, 900])
-    res = []
-    for cl, u in zip((ref, ora), unets):
-        cl(guide)
-        pred = u(x, t, ehs, cross_attention_kwargs={"scale": 0.8}).sample
-        loss = torch.nn.functional.mse_loss(pred, tgt)
-        loss.backward()
-        res.append((pred.detach(), float(loss), {n: p.grad.clone() for n, p in cl.named_parameters() if p.grad is not None}))
-    (pr, lr_, gr), (po, lo, go) = res
-    assert float((po - pr).abs().max()) <= 2e-5 * float(pr.abs().max()) and abs(lo - lr_) <= 1e-6 * abs(lr_)
-    assert set(go) == set(gr) and len(gr) > 50
-    for n in gr:
-        assert float((go[n] - gr[n]).abs().max()) <= 1e-4 * float(gr[n].abs().max()) + 1e-9, n
+    gold = GOLD["unet"][variant]
+    got = P.unet_case(MR, variant)
+    assert _close(got["pred"], gold["pred"], 2e-5) and abs(got["loss"] - gold["loss"]) <= 1e-6 * abs(gold["loss"])
+    assert set(got["grads"]) == set(gold["grads"]) and len(gold["grads"]) > 50
+    for n, b in gold["grads"].items():
+        assert _close(got["grads"][n], b, 1e-4, 1e-9), n
 
 
 @pytest.mark.parametrize("case", ["v1_stacked", "v2", "post_add", "concat"])
@@ -219,14 +103,3 @@ def test_oracle_matches_the_golden_vectors_generated_by_the_reference(case):
     assert got["grads"]["names"] == gold["grads"]["names"] and got["grad_norms"]["names"] == gold["grad_norms"]["names"]
     assert close(got["grads"]["flat"], gold["grads"]["flat"])
     assert float(((got["grad_norms"]["values"] - gold["grad_norms"]["values"]).abs() / gold["grad_norms"]["values"].clamp_min(1e-12)).max()) < 1e-3
-
-
-@needs_reference
-def test_committed_golden_vectors_are_what_the_reference_computes_now():
-    """Guards the fixture itself: regenerating one case from /root/reference/models.py gives the committed numbers."""
-    from tests.golden import make_reference_golden as G
-
-    gold = torch.load(G.OUT, weights_only=False)["v2"]
-    now = G.run_front_half(RI.reference_models(), "v2")
-    assert float((now["pred"] - gold["pred"]).abs().max()) <= 1e-6 * float(gold["pred"].abs().max())
-    assert float((now["grads"]["flat"] - gold["grads"]["flat"]).abs().max()) <= 1e-5 * float(gold["grads"]["flat"].abs().max())
